@@ -212,6 +212,22 @@ def workload_config(workload, cells, cycles, n_chips, inflight):
     return c
 
 
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(d, arrays):
+    """--dump-outputs: write each uint32 array as <d>/<name>.npy in float64 (exact for 32-bit words), so that two builds can be compared
+    output for output.  If all of them together exceed DUMP_CAP_BYTES, each keeps the same share of its words: a fixed, seeded sample of
+    its flattened positions, in increasing order."""
+    os.makedirs(d, exist_ok=True)
+    total = sum(a.size for a in arrays.values()) * 8
+    for name, a in arrays.items():
+        if total > DUMP_CAP_BYTES:
+            a = a.reshape(-1)
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, max(1, a.size * DUMP_CAP_BYTES // total), replace=False))]
+        np.save(os.path.join(d, name + ".npy"), a.astype(np.float64))
+
+
 def ref_kernels_leg(lib, n_cols, dev):
     """Head to head on this box: the REFERENCE's own CUDA kernels (oracle/_ref, compiled unmodified from sp1-gpu/crates/sys; launch
     shapes of its Rust host code) against this library's kernel-level entry points, on identical device buffers of the S2 commit
@@ -448,7 +464,13 @@ def main():
                          "per-shard H2D and a proof gather to rank 0 (strong scaling, BASELINE config 5)")
     ap.add_argument("--shards", type=int, default=64)
     ap.add_argument("--distinct", type=int, default=16, help="--job queue: number of distinct (heights, trace) sets the shards cycle over")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned to each in-flight caller of prove_shard (rank 0) as "
+                         "DIR/<name>.npy in float64: proof_words and challenger_state [inflight, ...] of the device-resident steps, "
+                         "e2e_proof_words and e2e_challenger_state of the e2e steps; at most 64 MB in all (larger: a fixed, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     if args.job == "queue":
@@ -519,6 +541,7 @@ def main():
     acc = {}
 
     def step(src, record=False, who=0):
+        """-> (proof words, final challenger state): what a caller of prove_shard receives"""
         l_, m_, p_ = provers[who]
         st = chal0.copy()
         proof = l_.prove_shard(m_, p_, src, heights, names, pv, st)
@@ -527,22 +550,20 @@ def main():
                 v = l_.phase_ms(n)
                 if v >= 0:
                     acc[n] = acc.get(n, 0.0) + v
-        return proof
+        return proof, st
 
     def run_steps(who, src, k, pipelined_upload, out):
         l_ = provers[who][0]
-        nbytes = 0
         if pipelined_upload:
             nxt = l_.upload_begin(src, 0)
             for i in range(k):
                 cur = nxt
                 if i + 1 < k:
                     nxt = l_.upload_begin(src, (i + 1) & 1)
-                nbytes = step(cur, record=True, who=who).nbytes
+                out[who] = step(cur, record=True, who=who)
         else:
             for _ in range(k):
-                nbytes = step(src, record=True, who=who).nbytes
-        out[who] = nbytes
+                out[who] = step(src, record=True, who=who)
 
     def sync_all():
         for l_, _, _ in provers:
@@ -552,14 +573,15 @@ def main():
     def timed(src, k, pipelined_upload=False):
         """k steps, each step = one shard per in-flight prover; pipelined_upload: src is the pinned host buffer, every shard's H2D
         goes through the library's double-buffered upload slots (C ABI sp1b200_upload_begin) so that the copy of the next shard
-        overlaps the proof of the current one — all copies are inside the timed region."""
+        overlaps the proof of the current one — all copies are inside the timed region.
+        -> (ms, launches, [(proof words, challenger state) of the last step, per in-flight prover])"""
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         if world > 1:
             dist.barrier()
         sync_all()
         l0 = sum(l_.launch_count() for l_, _, _ in provers)
         e0.record(stream)
-        out = [0] * len(provers)
+        out = [None] * len(provers)
         if len(provers) == 1:
             run_steps(0, src, k, pipelined_upload, out)
         else:
@@ -574,7 +596,7 @@ def main():
         if world > 1:
             dist.barrier()
         ms = SH.max_over_ranks(e0.elapsed_time(e1), dev)
-        return ms, sum(l_.launch_count() for l_, _, _ in provers) - l0, out[0]
+        return ms, sum(l_.launch_count() for l_, _, _ in provers) - l0, out
 
     if os.environ.get("SP1B200_PROFILE_RANGE") == "1":   # ncu --profile-from-start off: skip the torch trace synthesis and the setup
         torch.cuda.cudart().cudaProfilerStart()
@@ -590,13 +612,17 @@ def main():
     phases = {k: v / PHASE_REPS for k, v in acc.items()}
     acc.clear()
     with ClockSampler(local) as cs:
-        ms_dev, launches, proof_bytes = timed(d_main, args.steps)
+        ms_dev, launches, last_dev = timed(d_main, args.steps)
         acc.clear()
         if args.e2e_mode == "pipelined":
             for l_, _, _ in provers:
                 l_.upload_begin(h_main, 0); l_.upload_begin(h_main, 1); l_.sync()   # slot allocation is setup, not a step
-        ms_e2e, _, _ = timed(h_main, args.steps, pipelined_upload=(args.e2e_mode == "pipelined"))
+        ms_e2e, _, last_e2e = timed(h_main, args.steps, pipelined_upload=(args.e2e_mode == "pipelined"))
     clocks = cs.summary()
+    proof_bytes = last_dev[0][0].nbytes
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"proof_words": np.stack([p for p, _ in last_dev]), "challenger_state": np.stack([s for _, s in last_dev]),
+                                         "e2e_proof_words": np.stack([p for p, _ in last_e2e]), "e2e_challenger_state": np.stack([s for _, s in last_e2e])})
 
     total_cycles = cycles * world * len(provers)  # every rank proves `inflight` shards of the same size per step (weak scaling)
     value = total_cycles * args.steps / (ms_dev / 1e3)

@@ -1,5 +1,5 @@
-import sys, numpy as np
-sys.path.insert(0,'/root/repo')
+import os, sys, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from tests import oracle_lib as O, ref_lib as R
 rng=np.random.default_rng(301)
 for lg in (1,2):
