@@ -8,11 +8,6 @@
 #include <cstring>
 #include <cstdlib>
 
-sp1b200_err sp1b200_init_tables(sp1b200_ctx* ctx);
-sp1b200_err sp1b200_rs_encode_device(sp1b200_ctx*, const uint32_t*, uint64_t, uint32_t, uint32_t, uint32_t*);
-sp1b200_err sp1b200_permute_device(sp1b200_ctx*, uint32_t*, uint64_t);
-sp1b200_err sp1b200_merkle_commit_device(sp1b200_ctx*, const uint32_t*, uint64_t, uint32_t, uint32_t*, uint32_t*);
-
 static thread_local char g_err[1024];
 
 const char* sp1b200_set_error(const char* fmt, ...) {

@@ -156,6 +156,32 @@ struct DevBuf {
     ~DevBuf();
 };
 
+// stream-ordered scratch allocations from the context's pool, freed (stream-ordered) when the scope ends
+struct DevFree {
+    sp1b200_ctx* ctx;
+    std::vector<void*> ptrs;
+    explicit DevFree(sp1b200_ctx* c) : ctx(c) {}
+    ~DevFree() { for (void* p : ptrs) cudaFreeAsync(p, ctx->stream); }
+    sp1b200_err alloc(void** p, size_t bytes) {
+        SP1_CUDA(cudaMallocFromPoolAsync(p, bytes ? bytes : 4, ctx->pool, ctx->stream));
+        ptrs.push_back(*p);
+        return nullptr;
+    }
+};
+inline unsigned blocks_for(uint64_t n, unsigned bs = 256) { return (unsigned)((n + bs - 1) / bs); }
+
 bool sp1b200_is_device_ptr(const void* p);
 extern "C" int sp1b200_upload_acquire(sp1b200_ctx* c, const void* d_ptr);
 extern "C" void sp1b200_upload_release(sp1b200_ctx* c, int slot);
+
+// device-pointer implementations behind the C entry points, called across translation units (ntt.cu, merkle.cu)
+sp1b200_err sp1b200_init_tables(sp1b200_ctx* ctx);
+sp1b200_err sp1b200_rs_encode_device(sp1b200_ctx* ctx, const uint32_t* d_msg, uint64_t ncols, uint32_t log_h, uint32_t log_blowup,
+                                     uint32_t* d_out);
+sp1b200_err sp1b200_permute_device(sp1b200_ctx* ctx, uint32_t* d_states, uint64_t n);
+sp1b200_err sp1b200_merkle_commit_device(sp1b200_ctx* ctx, const uint32_t* d_mat, uint64_t width, uint32_t log_h, uint32_t* d_layers,
+                                         uint32_t* d_root_commit16);
+sp1b200_err sp1b200_merkle_tree_from_leaves_device(sp1b200_ctx* ctx, uint32_t* d_layers, uint32_t log_h, uint32_t width,
+                                                   uint32_t* d_root_commit16);
+sp1b200_err sp1b200_fri_tree_device(sp1b200_ctx* ctx, const uint32_t* d_cw, uint64_t m, uint32_t* d_layers, uint32_t log_leaves,
+                                    uint32_t* d_root_commit16, Mail mail);

@@ -9,10 +9,7 @@
 //    fused as "fix the previous variable + accumulate the next round's three sums";
 //  * once a layer's row variables are exhausted the remaining (interaction) variables range over <= 2^v <= a few
 //    thousand values, which the host transcript driver folds directly.
-#include "ctx.cuh"
-#include "challenger.cuh"
-#include "hostfield.hpp"
-#include "kb31.cuh"
+#include "sumcheck.cuh"
 #include <algorithm>
 #include <memory>
 #include <vector>
@@ -147,29 +144,6 @@ __device__ __forceinline__ void pair_sums(const Row4& x, const Row4& y, const Ex
     se = kb::ext_add(se, ees);
 }
 
-__device__ __forceinline__ void block_reduce3(Ext a, Ext b, Ext c, uint32_t* __restrict__ partial, const Mail& mail) {
-    // warp shuffles + one barrier (these kernels are latency-bound on the upper layers: a shared-memory tree costs 8 barriers)
-    __shared__ uint32_t red[12][8];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint32_t w[12];
-#pragma unroll
-    for (int l = 0; l < 4; l++) { w[l] = a.c[l]; w[4 + l] = b.c[l]; w[8 + l] = c.c[l]; }
-#pragma unroll
-    for (int k = 0; k < 12; k++) {
-        uint32_t v = w[k];
-#pragma unroll
-        for (int sft = 16; sft > 0; sft >>= 1) v = kb::add(v, __shfl_down_sync(0xffffffffu, v, sft));
-        if (lane == 0) red[k][warp] = v;
-    }
-    __syncthreads();
-    if (threadIdx.x < 12) {
-        uint32_t v = 0;
-        for (int q = 0; q < (int)(blockDim.x >> 5); q++) v = kb::add(v, red[threadIdx.x][q]);
-        partial[blockIdx.x * 12 + threadIdx.x] = v;
-    }
-    sp1_mail_done(mail);  // `partial` is the mailbox payload: the host transcript polls the flag (ctx.cuh)
-}
-
 // round 0 of a layer: sums straight from the fraction sequence. work item = (chip, k, row pair i)
 __global__ void __launch_bounds__(256) gkr_sum_seq_kernel(JobTable jobs, const uint32_t* __restrict__ num, const uint32_t* __restrict__ den,
                                                           const uint32_t* __restrict__ eq_int, const uint32_t* __restrict__ eq_row, Ext lambda,
@@ -184,7 +158,7 @@ __global__ void __launch_bounds__(256) gkr_sum_seq_kernel(JobTable jobs, const u
         Row4 x = row_from_seq(num, den, base, c.rows_in, 2 * i), y = row_from_seq(num, den, base, c.rows_in, 2 * i + 1);
         pair_sums(x, y, ldE(eq_int, c.int_off + k), ldE(eq_row, 2 * i), ldE(eq_row, 2 * i + 1), lambda, s0, sh, se);
     }
-    block_reduce3(s0, sh, se, partial, mail);
+    block_post_sums<3>({s0, sh, se}, partial, mail);
 }
 
 // fix the last row variable (input = fraction sequence or working arrays), write the working arrays of the next round and
@@ -222,7 +196,7 @@ __global__ void __launch_bounds__(256) gkr_fix_sum_kernel(JobTable jobs, const u
         }
         pair_sums(nr[0], nr[1], ldE(eq_int, c.int_off + k), ldE(eq_row_new, 2 * i), ldE(eq_row_new, 2 * i + 1), lambda, s0, sh, se);
     }
-    block_reduce3(s0, sh, se, partial, mail);
+    block_post_sums<3>({s0, sh, se}, partial, mail);
 }
 
 // ---- interaction variables (logup_poly.rs:118-176 + the generic round of sumcheck/src/prover.rs) -------------------------------
@@ -277,27 +251,9 @@ __global__ void __launch_bounds__(256) gkr_inter_round_kernel(const uint32_t* __
             for (int a = 0; a < 4; a++) { stE(payload, 3 + 2 * a, v[a][0]); stE(payload, 4 + 2 * a, v[a][1]); }
         }
     }
-    block_reduce3(s0, sh, se, payload, mail);
+    block_post_sums<3>({s0, sh, se}, payload, mail);
 }
 
-__global__ void gkr_eq_table_kernel(const uint32_t* __restrict__ point, int k, uint32_t* __restrict__ E) {
-    uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= ((uint64_t)1 << k)) return;
-    Ext acc = kb::ext_one();
-    for (int t = 0; t < k; t++) {
-        Ext x = kb::ext_load(point + 4 * t);
-        bool bit = (j >> (k - 1 - t)) & 1;
-        acc = kb::ext_mul(acc, bit ? x : kb::ext_sub(kb::ext_one(), x));
-    }
-    kb::ext_store(E + 4 * j, acc);
-}
-// E'[j] = E[2j] + alpha (E[2j+1] - E[2j])
-__global__ void gkr_fix_eq_kernel(const uint32_t* __restrict__ E, uint64_t n_out, Ext alpha, uint32_t* __restrict__ Eo) {
-    uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n_out) return;
-    Ext a = ldE(E, 2 * j), b = ldE(E, 2 * j + 1);
-    stE(Eo, j, kb::ext_add(a, kb::ext_mul(alpha, kb::ext_sub(b, a))));
-}
 // per-column openings of EVERY chip in two launches: out[c] = sum_{r < rows} eq[r] * col[r].
 // A block takes one chunk of OPEN_ROWS rows of one table (a chip's main or preprocessed columns), keeps its eq values in
 // registers and walks all the table's columns (coalesced column-major reads, 4 products per 64-bit accumulator and
@@ -370,16 +326,6 @@ __global__ void __launch_bounds__(256) gkr_open_reduce_kernel(const OpenJob* __r
     }
 }
 
-struct DevFree {
-    sp1b200_ctx* ctx; std::vector<void*> ptrs;
-    explicit DevFree(sp1b200_ctx* c) : ctx(c) {}
-    ~DevFree() { for (void* p : ptrs) cudaFreeAsync(p, ctx->stream); }
-    sp1b200_err alloc(void** p, size_t bytes) { SP1_CUDA(cudaMallocFromPoolAsync(p, bytes ? bytes : 4, ctx->pool, ctx->stream)); ptrs.push_back(*p); return nullptr; }
-};
-inline unsigned blocks_for(uint64_t n, unsigned bs = 256) { return (unsigned)((n + bs - 1) / bs); }
-
-inline Ext toExt(const E4& e) { return Ext{{e.c[0], e.c[1], e.c[2], e.c[3]}}; }
-
 // every read is bounds-checked against the end of the blob and every column against the chip's widths: a blob exported for another
 // chip set must become an error, not an out-of-bounds read on host or device
 const uint32_t* parse_vcol(const uint32_t* b, const uint32_t* end, HostInteractions& H, uint32_t main_w, uint32_t prep_w) {
@@ -422,19 +368,5 @@ void* sp1b200_parse_interactions(const uint32_t* b, const uint32_t* end, size_t 
     return H.release();
 }
 void sp1b200_free_interactions(void* p) { delete static_cast<HostInteractions*>(p); }
-
-extern "C" {
-
-// GkrProverImpl::prove_logup_gkr (crates/hypercube/src/logup_gkr/prover.rs:70-215).
-// d_main[k]/d_prep[k]: chip columns (column-major [w x h_heights[k]]), interactions from the machine blob.
-// h_replay_witness: the GKR grinding witness when params.grind_mode == 1.
-// Output words: n_out | numerator[n_out] ext | denominator[n_out] ext | n_rounds | per round {numerator_0, numerator_1,
-//   denominator_0, denominator_1 ext, sumcheck {n_polys, per poly {n_coeffs, coeffs}, claimed_sum, point, eval}} |
-//   evaluation point (max_log_row_count ext) | per chip {main openings, preprocessed openings} | witness
-sp1b200_err sp1b200_logup_gkr(sp1b200_ctx* ctx, const sp1b200_machine* m, const uint64_t* h_heights, const uint32_t* const* d_main,
-                              const uint32_t* const* d_prep, const uint32_t* h_replay_witness, uint32_t* h_chal, uint32_t* h_out, uint64_t cap,
-                              uint64_t* h_words);
-
-}
 
 #include "gkr_driver.inc"

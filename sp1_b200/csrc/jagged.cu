@@ -8,20 +8,10 @@
 // each sumcheck round after the first runs as ONE fused kernel (fix the previous variable + accumulate the next
 // round's sums) so the folded vectors are written once and read once; the branching-program sumcheck evaluates all
 // (column, node) pairs of a round in one launch.
-#include "ctx.cuh"
-#include "challenger.cuh"
-#include "hostfield.hpp"
-#include "kb31.cuh"
+#include "sumcheck.cuh"
 #include <algorithm>
 #include <memory>
 #include <vector>
-
-struct sp1b200_commit;
-extern "C" sp1b200_err sp1b200_stacked_commit(sp1b200_ctx*, const uint32_t*, uint64_t, int, uint32_t*, sp1b200_commit**);
-extern "C" void sp1b200_commit_free(sp1b200_ctx*, sp1b200_commit*);
-extern "C" sp1b200_err sp1b200_stacked_prove(sp1b200_ctx*, sp1b200_commit* const*, uint32_t, const uint32_t*, uint32_t, const uint32_t*,
-                                             uint32_t*, uint32_t*, uint64_t, uint64_t*);
-void host_poseidon2_permute(uint32_t* s16);
 
 #include "pcs.cuh"
 
@@ -47,32 +37,6 @@ void host_compress(const uint32_t* l, const uint32_t* r, uint32_t* out8) {
     for (int j = 0; j < 8; j++) { st[j] = l[j]; st[8 + j] = r[j]; }
     host_poseidon2_permute(st);
     for (int j = 0; j < 8; j++) out8[j] = st[j];
-}
-
-struct DevFree {
-    sp1b200_ctx* ctx;
-    std::vector<void*> ptrs;
-    explicit DevFree(sp1b200_ctx* c) : ctx(c) {}
-    ~DevFree() { for (void* p : ptrs) cudaFreeAsync(p, ctx->stream); }
-    sp1b200_err alloc(void** p, size_t bytes) {
-        SP1_CUDA(cudaMallocFromPoolAsync(p, bytes ? bytes : 4, ctx->pool, ctx->stream));
-        ptrs.push_back(*p);
-        return nullptr;
-    }
-};
-inline unsigned blocks_for(uint64_t n, unsigned bs = 256) { return (unsigned)((n + bs - 1) / bs); }
-
-// E[j] = prod_t (j_t ? x_t : 1 - x_t), point[0] <-> MSB of j
-__global__ void eq_table_kernel(const uint32_t* __restrict__ point, int k, uint32_t* __restrict__ E) {
-    uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= ((uint64_t)1 << k)) return;
-    Ext acc = kb::ext_one();
-    for (int t = 0; t < k; t++) {
-        Ext x = kb::ext_load(point + 4 * t);
-        bool bit = (j >> (k - 1 - t)) & 1;
-        acc = kb::ext_mul(acc, bit ? x : kb::ext_sub(kb::ext_one(), x));
-    }
-    kb::ext_store(E + 4 * j, acc);
 }
 
 // per-column claims: out[c] = sum_{r < rows} row_eq[r] * col[r]   (one block per column)
@@ -131,29 +95,6 @@ __device__ __forceinline__ uint32_t seg_load(const SegTable& t, uint64_t i) {
     return 0;
 }
 
-__device__ __forceinline__ void block_reduce2(Ext a, Ext b, uint32_t* __restrict__ partial, const Mail& mail) {
-    // warp shuffles + one barrier (the late rounds are latency-bound)
-    __shared__ uint32_t red[8][8];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint32_t w[8];
-#pragma unroll
-    for (int l = 0; l < 4; l++) { w[l] = a.c[l]; w[4 + l] = b.c[l]; }
-#pragma unroll
-    for (int k = 0; k < 8; k++) {
-        uint32_t v = w[k];
-#pragma unroll
-        for (int sft = 16; sft > 0; sft >>= 1) v = kb::add(v, __shfl_down_sync(0xffffffffu, v, sft));
-        if (lane == 0) red[k][warp] = v;
-    }
-    __syncthreads();
-    if (threadIdx.x < 8) {
-        uint32_t v = 0;
-        for (int q = 0; q < (int)(blockDim.x >> 5); q++) v = kb::add(v, red[threadIdx.x][q]);
-        partial[blockIdx.x * 8 + threadIdx.x] = v;
-    }
-    sp1_mail_done(mail);  // `partial` is the mailbox payload (ctx.cuh): the host transcript polls instead of copy + synchronise
-}
-
 // round 0: sum_j ext[2j]*base[2j]  and  sum_j (ext[2j]+ext[2j+1]) * (base[2j]+base[2j+1])   (base in F)
 __global__ void __launch_bounds__(256) hadamard_sum0_kernel(SegTable base, const uint32_t* __restrict__ ext, uint64_t npairs,
                                                             uint32_t* __restrict__ partial, Mail mail) {
@@ -164,7 +105,7 @@ __global__ void __launch_bounds__(256) hadamard_sum0_kernel(SegTable base, const
         s0 = kb::ext_add(s0, kb::ext_mul_base(e0, b0));
         sh = kb::ext_add(sh, kb::ext_mul_base(kb::ext_add(e0, e1), kb::add(b0, b1)));
     }
-    block_reduce2(s0, sh, partial, mail);
+    block_post_sums<2>({s0, sh}, partial, mail);
 }
 
 // fix the last variable of round 0 (base F -> EF) and accumulate round-1 sums
@@ -189,7 +130,7 @@ __global__ void __launch_bounds__(256) hadamard_fold0_kernel(SegTable base, cons
         s0 = kb::ext_add(s0, kb::ext_mul(ne[0], nb[0]));
         sh = kb::ext_add(sh, kb::ext_mul(kb::ext_add(ne[0], ne[1]), kb::ext_add(nb[0], nb[1])));
     }
-    block_reduce2(s0, sh, partial, mail);
+    block_post_sums<2>({s0, sh}, partial, mail);
 }
 
 // ---- round 0 without the materialised little polynomial ("factored" path) -------------------------------------------------------
@@ -205,12 +146,6 @@ __global__ void __launch_bounds__(256) hadamard_fold0_kernel(SegTable base, cons
 __device__ __forceinline__ uint32_t jp_column(const uint64_t* __restrict__ prefix, uint32_t ncols, uint32_t c, uint64_t i) {
     while (c + 1 < ncols && prefix[c + 1] <= i) c++;
     return c;
-}
-__global__ void __launch_bounds__(256) row_eq_fold_kernel(const uint32_t* __restrict__ row_eq, Ext alpha, uint64_t n_out, uint32_t* __restrict__ out) {
-    const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= n_out) return;
-    const Ext a = kb::ext_load(row_eq + 8 * k), b = kb::ext_load(row_eq + 8 * k + 4);
-    kb::ext_store(out + 4 * k, kb::ext_add(a, kb::ext_mul(alpha, kb::ext_sub(b, a))));
 }
 __global__ void __launch_bounds__(256) hadamard_sum0_fused_kernel(SegTable base, const uint64_t* __restrict__ prefix, uint32_t ncols,
                                                                   const uint32_t* __restrict__ start, const uint32_t* __restrict__ col_eq,
@@ -243,9 +178,9 @@ __global__ void __launch_bounds__(256) hadamard_sum0_fused_kernel(SegTable base,
         const Ext ce = kb::ext_load(col_eq + 4 * c);
         s0 = kb::ext_add(s0, kb::ext_mul(ce, t0)); sh = kb::ext_add(sh, kb::ext_mul(ce, th));
     }
-    block_reduce2(s0, sh, partial, mail);
+    block_post_sums<2>({s0, sh}, partial, mail);
 }
-// fix the last variable of round 0 in product form and accumulate round-1 sums; roweq2 = row_eq folded by alpha (row_eq_fold_kernel)
+// fix the last variable of round 0 in product form and accumulate round-1 sums; roweq2 = row_eq folded by alpha (fix_last_kernel)
 __global__ void __launch_bounds__(256) hadamard_fold0_fused_kernel(SegTable base, const uint64_t* __restrict__ prefix, uint32_t ncols,
                                                                    const uint32_t* __restrict__ start, const uint32_t* __restrict__ col_eq,
                                                                    const uint32_t* __restrict__ roweq2, uint64_t area, uint64_t nout_pairs, Ext alpha,
@@ -272,7 +207,7 @@ __global__ void __launch_bounds__(256) hadamard_fold0_fused_kernel(SegTable base
         s0 = kb::ext_add(s0, kb::ext_mul(ne[0], nb[0]));
         sh = kb::ext_add(sh, kb::ext_mul(kb::ext_add(ne[0], ne[1]), kb::ext_add(nb[0], nb[1])));
     }
-    block_reduce2(s0, sh, partial, mail);
+    block_post_sums<2>({s0, sh}, partial, mail);
 }
 
 // rounds >= 1: fix the last variable (EF -> EF) and accumulate the next round's sums
@@ -298,7 +233,7 @@ __global__ void __launch_bounds__(256) hadamard_fold_kernel(const uint32_t* __re
         s0 = kb::ext_add(s0, kb::ext_mul(ne[0], nb[0]));
         sh = kb::ext_add(sh, kb::ext_mul(kb::ext_add(ne[0], ne[1]), kb::ext_add(nb[0], nb[1])));
     }
-    block_reduce2(s0, sh, partial, mail);
+    block_post_sums<2>({s0, sh}, partial, mail);
 }
 
 // ---- branching program (slop/crates/jagged/src/poly.rs:136-175, 384-470) ---------------------------------------
@@ -542,20 +477,12 @@ inline void interp_0_1_half(const E4& y0, const E4& y1, const E4& yh, E4 c[3]) {
 }
 inline E4 eval3(const E4 c[3], const E4& x) { return (c[2] * x + c[1]) * x + c[0]; }
 
-sp1b200_err sum_partials(sp1b200_ctx* ctx, const uint32_t* d_partial, unsigned nblk, E4& a, E4& b) {
+sp1b200_err sum_partials(sp1b200_ctx* ctx, const uint32_t* d_partial, unsigned nblk, E4 (&out)[2]) {
     std::vector<uint32_t> h((size_t)nblk * 8);
     SP1_CUDA(cudaMemcpyAsync(h.data(), d_partial, h.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
     SP1_CUDA(cudaStreamSynchronize(ctx->stream));
-    a = E4(); b = E4();
-    for (unsigned k = 0; k < nblk; k++) { a = a + E4::load(&h[8 * k]); b = b + E4::load(&h[8 * k + 4]); }
-    return nullptr;
-}
-// same sums from the mailbox payload of the posting kernel with sequence number `seq` (8 words per block)
-sp1b200_err sum_mail(sp1b200_ctx* ctx, uint32_t seq, unsigned nblk, E4& a, E4& b) {
-    SP1_TRY(sp1b200_mail_wait(ctx, seq));
-    const uint32_t* h = sp1b200_mail_host(ctx);
-    a = E4(); b = E4();
-    for (unsigned k = 0; k < nblk; k++) { a = a + E4::load(&h[8 * k]); b = b + E4::load(&h[8 * k + 4]); }
+    out[0] = E4(); out[1] = E4();
+    for (unsigned k = 0; k < nblk; k++) { out[0] = out[0] + E4::load(&h[8 * k]); out[1] = out[1] + E4::load(&h[8 * k + 4]); }
     return nullptr;
 }
 
@@ -735,8 +662,7 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
     { uint64_t e = 0; for (uint32_t r = 0; r < n_rounds; r++) { seg.ptr[r] = rounds[r]->d_dense; e += rounds[r]->padded_area; seg.end[r] = e; } }
 
     // ---- Hadamard sumcheck (lambda = 1, t = 1) ---------------------------------------------------------------------
-    std::vector<uint32_t> sc_words;     // univariate polys
-    std::vector<E4> point;              // most recent challenge first
+    SumcheckProof sc;
     E4 round_claim = claim;
     PhaseTimer t_sc(ctx, "jagged.sumcheck");
     auto grid_for = [&](uint64_t n) { unsigned g = blocks_for(n); return g > MAXB ? MAXB : (g ? g : 1u); };
@@ -745,7 +671,7 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
     uint32_t prev_seq = 0;
     for (uint32_t rd = 0; rd < lm; rd++) {
         const uint64_t n = N >> rd;  // current length
-        E4 e0, eh;
+        E4 s[2];  // the sum at 0, 4 x the sum at 1/2
         unsigned g;
         if (rd == 0) {
             g = grid_for(n / 2);
@@ -759,28 +685,22 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
             } else {
                 SP1_LAUNCH(ctx, hadamard_sum0_kernel, g, 256, 0, seg, cur_e, n / 2, d_partial, mail);
             }
-            SP1_TRY(sum_mail(ctx, mail.seq, g, e0, eh));
+            SP1_TRY(mail_sums(ctx, mail.seq, g, s));
         } else {
-            SP1_TRY(sum_mail(ctx, prev_seq, prev_g, e0, eh));  // accumulated by the previous fold launch
+            SP1_TRY(mail_sums(ctx, prev_seq, prev_g, s));  // accumulated by the previous fold launch
         }
-        E4 e1 = round_claim - e0;
         E4 c[3];
-        interp_0_1_half(e0, e1, eh * hf::inv(hf::to_monty(4)), c);
-        for (int i = 0; i < 3; i++) ch.observe_n(c[i].c, 4);
-        uint32_t three = 3;
-        sc_words.push_back(three);
-        for (int i = 0; i < 3; i++) sc_words.insert(sc_words.end(), c[i].c, c[i].c + 4);
-        E4 alpha; ch.sample_ext(alpha.c);
-        point.insert(point.begin(), alpha);
+        interp_0_1_half(s[0], round_claim - s[0], s[1] * hf::inv(hf::to_monty(4)), c);
+        const E4 alpha = sc.round(ch, c, 3);
         round_claim = eval3(c, alpha);
         // fix the variable; the same launch accumulates the next round's sums (unless this was the last round)
         const uint64_t nout = n / 2;
-        Ext da{{alpha.c[0], alpha.c[1], alpha.c[2], alpha.c[3]}};
+        const Ext da = to_ext(alpha);
         g = grid_for((nout + 1) / 2);
         const Mail mail = sp1b200_mail_next(ctx); prev_seq = mail.seq;
         if (rd == 0) {
             if (factored) {
-                SP1_LAUNCH(ctx, row_eq_fold_kernel, blocks_for((uint64_t)1 << (mlr - 1)), 256, 0, d_roweq, da, (uint64_t)1 << (mlr - 1), d_roweq2);
+                SP1_LAUNCH(ctx, fix_last_kernel, blocks_for((uint64_t)1 << (mlr - 1)), 256, 0, d_roweq, (uint64_t)1 << (mlr - 1), da, d_roweq2);
                 SP1_LAUNCH(ctx, hadamard_fold0_fused_kernel, g, 256, 0, seg, d_prefix, (uint32_t)total_cols, d_jp_start, d_coleq, d_roweq2, prefix.back(),
                            (nout + 1) / 2, da, nxt_b, nxt_e, d_partial, nout, mail);
             } else {
@@ -801,9 +721,8 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
     t_sc.stop();
 
     // ---- jagged evaluation (branching program) sumcheck --------------------------------------------------------------
-    std::vector<uint32_t> je_words;
-    std::vector<E4> rhos;
-    E4 je_claimed, je_eval;
+    SumcheckProof je;
+    E4 je_claimed[2], je_eval;
     {
         PhaseTimer t(ctx, "jagged.eval_sumcheck");
         const uint32_t dim = 2 * (lm + 1);
@@ -823,7 +742,7 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
         auto lsb = [](const std::vector<E4>& p, uint32_t i) { return p.size() <= i ? E4() : p[p.size() - 1 - i]; };
         if (mlr > hl) return sp1b200_set_error("jagged_prove: max_log_row_count %u exceeds log_m+1 = %u (unsupported shape)", mlr, hl);
         for (uint32_t l = 0; l < hl; l++) {
-            E4 zr = lsb(z_row, l), zi = lsb(point, l), one = E4::one();
+            E4 zr = lsb(z_row, l), zi = lsb(sc.point, l), one = E4::one();
             E4 p = zr * zi;
             E4 e11 = p, e10 = zr - p, e01 = zi - p, e00 = one - zr - e01;
             e00.store(&ri[l * 16]); e01.store(&ri[l * 16 + 4]); e10.store(&ri[l * 16 + 8]); e11.store(&ri[l * 16 + 12]);
@@ -842,14 +761,12 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
         std::vector<E4> ones(nk, E4::one());
         SP1_CUDA(cudaMemcpyAsync(d_inter, ones.data(), (size_t)nk * 16, cudaMemcpyHostToDevice, st));
         const E4 half = E4::from_base(hf::inv(hf::to_monty(2)));
-        Ext dhalf{{half.c[0], 0, 0, 0}};
+        const Ext dhalf = to_ext(half);
         // claimed sum = full evaluation at the boolean prefix sums (full_jagged_little_polynomial_evaluation, poly.rs:183-232)
-        E4 dummy;
         SP1_LAUNCH(ctx, bp_round_kernel, nblk, 128, 0, d_bits, nk, dim, dim, 0, d_rhos, d_ri, d_zc, d_inter, dhalf, d_part);
-        SP1_TRY(sum_partials(ctx, d_part, nblk, je_claimed, dummy));
-        ch.observe_n(je_claimed.c, 4);
-        E4 cl = je_claimed;
-        je_words.push_back(dim);
+        SP1_TRY(sum_partials(ctx, d_part, nblk, je_claimed));
+        ch.observe_n(je_claimed[0].c, 4);
+        E4 cl = je_claimed[0];
         // prefix / suffix states (see bp_suffix_kernel): T for the first half now, rebuilt once when the second half starts
         uint32_t *d_T, *d_P, *d_rho_pos;
         SP1_TRY(mem.alloc((void**)&d_T, (size_t)(hl + 2) * nk * 64));
@@ -868,20 +785,14 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
             const Mail mail = sp1b200_mail_next(ctx);
             SP1_LAUNCH(ctx, bp_round2_kernel, nblk, 128, 0, d_bits, nk, dim, round, d_rho_pos, d_ri, d_zc, d_inter, d_P, d_T, dhalf,
                        bp_mail ? sp1b200_mail_dev(ctx) : d_part, bp_mail ? mail : Mail{nullptr, nullptr, 0});
-            E4 y0, yh;
-            if (bp_mail) SP1_TRY(sum_mail(ctx, mail.seq, nblk, y0, yh));
-            else SP1_TRY(sum_partials(ctx, d_part, nblk, y0, yh));
-            E4 y1 = cl - y0;
+            E4 y[2];  // values at 0 and 1/2
+            if (bp_mail) SP1_TRY(mail_sums(ctx, mail.seq, nblk, y));
+            else SP1_TRY(sum_partials(ctx, d_part, nblk, y));
             E4 c[3];
-            interp_0_1_half(y0, y1, yh, c);
-            for (int i = 0; i < 3; i++) ch.observe_n(c[i].c, 4);
-            je_words.push_back(3);
-            for (int i = 0; i < 3; i++) je_words.insert(je_words.end(), c[i].c, c[i].c + 4);
-            E4 alpha; ch.sample_ext(alpha.c);
-            rhos.insert(rhos.begin(), alpha);
+            interp_0_1_half(y[0], cl - y[0], y[1], c);
+            const E4 alpha = je.round(ch, c, 3);
             cl = eval3(c, alpha);
-            Ext da{{alpha.c[0], alpha.c[1], alpha.c[2], alpha.c[3]}};
-            SP1_LAUNCH(ctx, bp_update_kernel, blocks_for(nk, 128), 128, 0, d_bits, nk, dim, round, da, d_rho_pos, d_ri, d_inter, d_P);
+            SP1_LAUNCH(ctx, bp_update_kernel, blocks_for(nk, 128), 128, 0, d_bits, nk, dim, round, to_ext(alpha), d_rho_pos, d_ri, d_inter, d_P);
         }
         je_eval = cl;
         t.stop();
@@ -893,25 +804,16 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
     ch.store(chal);
     std::vector<sp1b200_commit*> handles;
     for (uint32_t r = 0; r < n_rounds; r++) handles.push_back(rounds[r]->stacked);
-    std::vector<uint32_t> pt(point.size() * 4);
-    for (size_t i = 0; i < point.size(); i++) point[i].store(&pt[4 * i]);
+    std::vector<uint32_t> pt(sc.point.size() * 4);
+    for (size_t i = 0; i < sc.point.size(); i++) sc.point[i].store(&pt[4 * i]);
     // the stacked proof is written straight into the caller's buffer; the jagged sections are appended after it
     uint64_t nw = 0;
-    SP1_TRY(sp1b200_stacked_prove(ctx, handles.data(), n_rounds, pt.data(), (uint32_t)point.size(), h_replay, chal, h_proof, cap, &nw));
+    SP1_TRY(sp1b200_stacked_prove(ctx, handles.data(), n_rounds, pt.data(), (uint32_t)sc.point.size(), h_replay, chal, h_proof, cap, &nw));
     std::vector<uint32_t> proof;
     auto put = [&](const uint32_t* p, size_t n) { proof.insert(proof.end(), p, p + n); };
     auto put1 = [&](uint32_t v) { proof.push_back(v); };
-    // sumcheck proof
-    put1(lm);
-    put(sc_words.data(), sc_words.size());
-    put(claim.c, 4);
-    put(pt.data(), pt.size());
-    put(round_claim.c, 4);
-    // jagged eval proof
-    put(je_words.data(), je_words.size());
-    put(je_claimed.c, 4);
-    for (auto& x : rhos) put(x.c, 4);
-    put(je_eval.c, 4);
+    sc.emit(proof, claim, round_claim);
+    je.emit(proof, je_claimed[0], je_eval);
     for (uint32_t r = 0; r < n_rounds; r++) {
         put1((uint32_t)rounds[r]->row_counts.size());
         for (size_t t = 0; t < rounds[r]->row_counts.size(); t++) { put1((uint32_t)rounds[r]->row_counts[t]); put1((uint32_t)rounds[r]->col_counts[t]); }

@@ -201,8 +201,6 @@ sp1b200_err sp1b200_permute_device(sp1b200_ctx* ctx, uint32_t* d_states, uint64_
     return nullptr;
 }
 
-sp1b200_err sp1b200_merkle_tree_from_leaves_device(sp1b200_ctx* ctx, uint32_t* d_layers, uint32_t log_h, uint32_t width, uint32_t* d_root_commit16);
-
 // d_layers: (2^(log_h+1) - 1) digests; d_root_commit16: 16 words (root, commitment)
 sp1b200_err sp1b200_merkle_commit_device(sp1b200_ctx* ctx, const uint32_t* d_mat, uint64_t width, uint32_t log_h,
                                          uint32_t* d_layers, uint32_t* d_root_commit16) {

@@ -8,19 +8,11 @@
 // fold_even_odd rule, pinned by slop/crates/basefold/src/verifier.rs:309-386) instead of re-encoding the folded
 // MLE each round, the eq table for fixed_at_zero is built once and halved per round, and the PoW witnesses are
 // the deterministic minimum (or replayed).
-#include "ctx.cuh"
-#include "challenger.cuh"
-#include "hostfield.hpp"
-#include "kb31.cuh"
+#include "sumcheck.cuh"
 #include "poseidon2.cuh"
 #include <array>
 #include <memory>
 #include <vector>
-
-sp1b200_err sp1b200_rs_encode_device(sp1b200_ctx*, const uint32_t*, uint64_t, uint32_t, uint32_t, uint32_t*);
-sp1b200_err sp1b200_merkle_commit_device(sp1b200_ctx*, const uint32_t*, uint64_t, uint32_t, uint32_t*, uint32_t*);
-sp1b200_err sp1b200_merkle_tree_from_leaves_device(sp1b200_ctx*, uint32_t*, uint32_t, uint32_t, uint32_t*);
-sp1b200_err sp1b200_fri_tree_device(sp1b200_ctx*, const uint32_t*, uint64_t, uint32_t*, uint32_t, uint32_t*, Mail);
 
 struct sp1b200_commit {
     uint64_t ncols = 0;
@@ -40,20 +32,6 @@ __device__ __forceinline__ uint32_t root_pow(const uint32_t* __restrict__ TH, co
     uint32_t hi = __ldg(TH + (e >> 12));
     uint32_t lo = e & 4095u;
     return lo ? kb::mul(hi, __ldg(TL + lo)) : hi;
-}
-
-// E[j] = prod_t (j_t ? x_t : 1 - x_t), point[0] <-> MSB of j
-__global__ void eq_table_kernel(const uint32_t* __restrict__ point, int k, uint32_t* __restrict__ E) {
-    uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= ((uint64_t)1 << k)) return;
-    Ext acc = kb::ext_one();
-    for (int t = 0; t < k; t++) {
-        Ext x = kb::ext_load(point + 4 * t);
-        bool bit = (j >> (k - 1 - t)) & 1;
-        Ext f = bit ? x : kb::ext_sub(kb::ext_one(), x);
-        acc = kb::ext_mul(acc, f);
-    }
-    kb::ext_store(E + 4 * j, acc);
 }
 
 // out[i] (+)= sum_c coeff[c] * cols[c][i]   ; out as Ext AoS [h]
@@ -151,13 +129,6 @@ __global__ void __launch_bounds__(256) dot_even_kernel(const uint32_t* __restric
     if (threadIdx.x < 4) partial[blockIdx.x * 4 + threadIdx.x] = red[threadIdx.x][0];
 }
 
-// E'[j] = E[2j] + E[2j+1]  (drops the last coordinate of the eq point)
-__global__ void halve_eq_kernel(const uint32_t* __restrict__ E, uint64_t n_out, uint32_t* __restrict__ Eo) {
-    uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n_out) return;
-    kb::ext_store(Eo + 4 * j, kb::ext_add(kb::ext_load(E + 8 * j), kb::ext_load(E + 8 * j + 4)));
-}
-
 // mle'[j] = mle[2j] + beta * mle[2j+1]
 __global__ void fold_mle_kernel(const uint32_t* __restrict__ mle, uint64_t n_out, Ext beta, uint32_t* __restrict__ out) {
     uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -218,20 +189,6 @@ __global__ void gather_fri_values_kernel(const uint32_t* __restrict__ cw, uint64
     uint32_t q = t >> 3, w = t & 7;
     out[t] = cw[(w & 3) * m + 2 * (uint64_t)idx[q] + (w >> 2)];
 }
-
-struct DevFree {
-    sp1b200_ctx* ctx;
-    std::vector<void*> ptrs;
-    explicit DevFree(sp1b200_ctx* c) : ctx(c) {}
-    ~DevFree() { for (void* p : ptrs) cudaFreeAsync(p, ctx->stream); }
-    sp1b200_err alloc(void** p, size_t bytes) {
-        SP1_CUDA(cudaMallocFromPoolAsync(p, bytes ? bytes : 4, ctx->pool, ctx->stream));
-        ptrs.push_back(*p);
-        return nullptr;
-    }
-};
-
-inline unsigned blocks_for(uint64_t n, unsigned bs = 256) { return (unsigned)((n + bs - 1) / bs); }
 
 }  // namespace
 
@@ -431,12 +388,9 @@ sp1b200_err sp1b200_stacked_prove(sp1b200_ctx* ctx, sp1b200_commit* const* round
         fri_commits.insert(fri_commits.end(), rc + 8, rc + 16);
         memcpy(fri_roots[r].data(), rc, 32);
         E4 beta; ch.sample_ext(beta.c);
-        Ext dbeta{{beta.c[0], beta.c[1], beta.c[2], beta.c[3]}};
-        E4 bh = beta * half;
-        Ext dbh{{bh.c[0], bh.c[1], bh.c[2], bh.c[3]}};
-        SP1_LAUNCH(ctx, fold_codeword_kernel, blocks_for(m_cur / 2), 256, 0, cw_ptr[r], (int)(log_h + b - r), dbh, half, ctx->d_TH,
-                   ctx->d_TL, cw_ptr[r + 1]);
-        SP1_LAUNCH(ctx, fold_mle_kernel, blocks_for(n_cur / 2), 256, 0, cur_mle, n_cur / 2, dbeta, nxt_mle);
+        SP1_LAUNCH(ctx, fold_codeword_kernel, blocks_for(m_cur / 2), 256, 0, cw_ptr[r], (int)(log_h + b - r), to_ext(beta * half), half,
+                   ctx->d_TH, ctx->d_TL, cw_ptr[r + 1]);
+        SP1_LAUNCH(ctx, fold_mle_kernel, blocks_for(n_cur / 2), 256, 0, cur_mle, n_cur / 2, to_ext(beta), nxt_mle);
         std::swap(cur_mle, nxt_mle);
         claim = zero_val + beta * one_val;
     }

@@ -13,14 +13,6 @@
 #include <vector>
 
 extern "C" {
-sp1b200_err sp1b200_jagged_commit(sp1b200_ctx*, const uint32_t*, uint32_t, const uint64_t*, const uint64_t*, int, uint32_t*, sp1b200_jagged_round**);
-void sp1b200_jagged_round_free(sp1b200_ctx*, sp1b200_jagged_round*);
-sp1b200_err sp1b200_jagged_prove(sp1b200_ctx*, sp1b200_jagged_round* const*, uint32_t, const uint32_t*, const uint32_t*, const uint32_t*, uint32_t*,
-                                 uint32_t*, uint64_t, uint64_t*);
-sp1b200_err sp1b200_logup_gkr(sp1b200_ctx*, const sp1b200_machine*, const uint64_t*, const uint32_t* const*, const uint32_t* const*, const uint32_t*,
-                              uint32_t*, uint32_t*, uint64_t, uint64_t*);
-sp1b200_err sp1b200_zerocheck(sp1b200_ctx*, const sp1b200_machine*, const uint64_t*, const uint32_t* const*, const uint32_t* const*, const uint32_t*,
-                              uint32_t, const uint32_t*, const uint32_t*, const uint32_t*, const uint32_t*, uint32_t*, uint32_t*, uint64_t, uint64_t*);
 
 // Proof words: [5][len_0..len_4] then the sections
 //   0 main commitment (8) | 1 LogUp-GKR proof (sp1b200_logup_gkr words) | 2 zerocheck proof + opened values (sp1b200_zerocheck words) |

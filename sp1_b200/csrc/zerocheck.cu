@@ -10,10 +10,7 @@
 // opening-batching term  sum_j gamma^j col_j  is evaluated once per row pair (at 0 and 1) instead of at every node.
 // The eq table is built once and halved per round; trace columns stay column-major (base field in round 0, EF afterwards);
 // geq / padded-row corrections and the 5-node interpolation run on the host from nine EF partial sums per chip.
-#include "ctx.cuh"
-#include "challenger.cuh"
-#include "hostfield.hpp"
-#include "kb31.cuh"
+#include "sumcheck.cuh"
 #include <algorithm>
 #include <memory>
 #include <vector>
@@ -315,23 +312,6 @@ __global__ void __launch_bounds__(256) zc_batch0_kernel(const ZcFixJob* __restri
     kb::ext_store(job.out + 4 * i, kb::ext_add(sa, kb::ext_mul(alpha, sd)));
 }
 
-__global__ void zc_eq_table_kernel(const uint32_t* __restrict__ point, int k, uint32_t* __restrict__ E) {
-    uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= ((uint64_t)1 << k)) return;
-    Ext acc = kb::ext_one();
-    for (int t = 0; t < k; t++) {
-        Ext x = kb::ext_load(point + 4 * t);
-        bool bit = (j >> (k - 1 - t)) & 1;
-        acc = kb::ext_mul(acc, bit ? x : kb::ext_sub(kb::ext_one(), x));
-    }
-    kb::ext_store(E + 4 * j, acc);
-}
-__global__ void zc_halve_eq_kernel(const uint32_t* __restrict__ E, uint64_t n_out, uint32_t* __restrict__ Eo) {
-    uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n_out) return;
-    kb::ext_store(Eo + 4 * j, kb::ext_add(kb::ext_load(E + 8 * j), kb::ext_load(E + 8 * j + 4)));
-}
-
 // host interpreter on the all-zero row (padded_row_adjustment, shard.rs:520-537): Σ powers[alpha_idx] * reg
 E4 host_eval_zero_row(const HostProg& p, const uint32_t* pv, const std::vector<E4>& powers, uint32_t n_regs) {
     std::vector<uint32_t> regs(n_regs ? n_regs : 1, 0);
@@ -360,14 +340,6 @@ struct VGeq {
     }
     E4 at(uint64_t idx) const { return idx < threshold ? E4() : (idx == threshold ? eq_c + geq_c : geq_c); }
 };
-
-struct DevFree {
-    sp1b200_ctx* ctx; std::vector<void*> ptrs;
-    explicit DevFree(sp1b200_ctx* c) : ctx(c) {}
-    ~DevFree() { for (void* p : ptrs) cudaFreeAsync(p, ctx->stream); }
-    sp1b200_err alloc(void** p, size_t bytes) { SP1_CUDA(cudaMallocFromPoolAsync(p, bytes ? bytes : 4, ctx->pool, ctx->stream)); ptrs.push_back(*p); return nullptr; }
-};
-inline unsigned blocks_for(uint64_t n, unsigned bs = 256) { return (unsigned)((n + bs - 1) / bs); }
 
 }  // namespace
 
@@ -557,7 +529,7 @@ sp1b200_err sp1b200_zerocheck(sp1b200_ctx* ctx, const sp1b200_machine* m, const 
     SP1_CUDA(cudaMemcpyAsync(d_point, h_gkr_point, mlr * 16, cudaMemcpyHostToDevice, st));
     SP1_TRY(mem.alloc((void**)&d_E[0], ((size_t)16 << (mlr - 1))));
     SP1_TRY(mem.alloc((void**)&d_E[1], ((size_t)16 << (mlr > 1 ? mlr - 2 : 0))));
-    SP1_LAUNCH(ctx, zc_eq_table_kernel, blocks_for((uint64_t)1 << (mlr - 1)), 256, 0, d_point, (int)mlr - 1, d_E[0]);
+    SP1_LAUNCH(ctx, eq_table_kernel, blocks_for((uint64_t)1 << (mlr - 1)), 256, 0, d_point, (int)mlr - 1, d_E[0]);
     int ecur = 0;
 
     // ---- the whole launch plan is known up front (heights halve deterministically): job tables of every round, one upload ----
@@ -683,9 +655,7 @@ sp1b200_err sp1b200_zerocheck(sp1b200_ctx* ctx, const sp1b200_machine* m, const 
     std::vector<E4> round_claims(nchips);
     E4 claimed_sum;
     for (size_t k = 0; k < nchips; k++) { round_claims[k] = E4::load(h_claims + 4 * k); claimed_sum = claimed_sum * lambda + round_claims[k]; }
-    std::vector<uint32_t> words;
-    words.push_back(mlr);
-    std::vector<E4> point;
+    SumcheckProof sc;
     std::vector<E4> ys((size_t)nchips * 4);  // per chip: round polynomial values at the nodes 0, 1, 2, 4
     std::vector<uint32_t> hs((size_t)max_jobs * 36);
     std::vector<E4> chip_sums(nchips * 9);
@@ -752,12 +722,8 @@ sp1b200_err sp1b200_zerocheck(sp1b200_ctx* ctx, const sp1b200_machine* m, const 
         }
         E4 rlc[5];
         for (int c5 = 0; c5 < 5; c5++) for (int i = 0; i < 4; i++) rlc[c5] = rlc[c5] + basis[i][c5] * Y[i];
-        for (auto& c : rlc) ch.observe_n(c.c, 4);
-        words.push_back(5);
-        for (auto& c : rlc) words.insert(words.end(), c.c, c.c + 4);
-        E4 a; ch.sample_ext(a.c);
-        point.insert(point.begin(), a);
-        const Ext da{{a.c[0], a.c[1], a.c[2], a.c[3]}};
+        const E4 a = sc.round(ch, rlc, 5);
+        const Ext da = to_ext(a);
         if (R.fix_jobs) {
             if (rd == 0) {
                 SP1_LAUNCH(ctx, zc_fix_kernel<uint32_t>, R.fix_blocks, 256, 0, d_fjobs + R.fix0, (int)R.fix_jobs, da);
@@ -778,15 +744,14 @@ sp1b200_err sp1b200_zerocheck(sp1b200_ctx* ctx, const sp1b200_machine* m, const 
         }
         if (rd + 1 < mlr) {
             const uint64_t n_out = (uint64_t)1 << (mlr - 2 - rd);
-            SP1_LAUNCH(ctx, zc_halve_eq_kernel, blocks_for(n_out), 256, 0, d_E[ecur], n_out, d_E[ecur ^ 1]);
+            SP1_LAUNCH(ctx, halve_eq_kernel, blocks_for(n_out), 256, 0, d_E[ecur], n_out, d_E[ecur ^ 1]);
             ecur ^= 1;
         }
     }
     E4 final_eval;
     for (auto& c : round_claims) final_eval = final_eval * lambda + c;
-    words.insert(words.end(), claimed_sum.c, claimed_sum.c + 4);
-    for (auto& x : point) words.insert(words.end(), x.c, x.c + 4);
-    words.insert(words.end(), final_eval.c, final_eval.c + 4);
+    std::vector<uint32_t> words;
+    sc.emit(words, claimed_sum, final_eval);
     // opened values: one EF row per chip (main columns then preprocessed, zeros for absent chips), fetched with one copy;
     // observed and emitted prep-first as the reference does
     std::vector<uint32_t> fin((wsum ? wsum : 1) * 4);
