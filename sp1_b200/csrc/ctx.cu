@@ -71,7 +71,6 @@ static sp1b200_err ctx_init(sp1b200_ctx* c, int device, const sp1b200_params* pa
     c->device = device;
     c->num_sms = prop.multiProcessorCount;
     if (params) c->params = *params; else sp1b200_default_core_params(&c->params);
-    { const char* g = getenv("SP1B200_GENERIC_NTT"); c->force_generic_ntt = g && g[0] == '1'; }
     SP1_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
     SP1_CUDA(cudaEventCreate(&c->ev0));
     SP1_CUDA(cudaEventCreate(&c->ev1));

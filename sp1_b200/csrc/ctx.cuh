@@ -23,7 +23,6 @@ struct sp1b200_ctx {
     uint32_t* d_TH = nullptr;
     uint32_t* d_TL = nullptr;
     uint64_t launches = 0;
-    bool force_generic_ntt = false;  // SP1B200_GENERIC_NTT=1: reference (slow) kernels, used to cross-check the fast path
     std::map<std::string, float> phase_ms;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     // mailbox: pinned + mapped host memory the round kernels write their few result words into, followed by a sequence flag;

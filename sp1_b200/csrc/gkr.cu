@@ -254,78 +254,6 @@ __global__ void __launch_bounds__(256) gkr_inter_round_kernel(const uint32_t* __
     block_post_sums<3>({s0, sh, se}, payload, mail);
 }
 
-// per-column openings of EVERY chip in two launches: out[c] = sum_{r < rows} eq[r] * col[r].
-// A block takes one chunk of OPEN_ROWS rows of one table (a chip's main or preprocessed columns), keeps its eq values in
-// registers and walks all the table's columns (coalesced column-major reads, 4 products per 64-bit accumulator and
-// reduction); per-column block sums go to partial[(blk_of_table)][col], a second launch adds the chunks.
-constexpr int OPEN_ROWS_PER_THREAD = 16;
-constexpr int OPEN_ROWS = 256 * OPEN_ROWS_PER_THREAD;
-struct OpenJob { const uint32_t* cols; uint64_t h; uint32_t w, blk_start, nblk, out_col; uint64_t part_off; };
-
-template <class J>
-__device__ __forceinline__ int open_find_job(const J* __restrict__ jobs, int n, uint32_t blk) {
-    int lo = 0, hi = n - 1;
-    while (lo < hi) {
-        int mid = (lo + hi + 1) >> 1;
-        if (jobs[mid].blk_start <= blk) lo = mid; else hi = mid - 1;
-    }
-    return lo;
-}
-
-__global__ void __launch_bounds__(256) gkr_open_partial_kernel(const OpenJob* __restrict__ jobs, int n_jobs, const uint32_t* __restrict__ eq,
-                                                               uint32_t* __restrict__ partial) {
-    const OpenJob job = jobs[open_find_job(jobs, n_jobs, blockIdx.x)];
-    const uint32_t chunk = blockIdx.x - job.blk_start;
-    const uint64_t row0 = (uint64_t)chunk * OPEN_ROWS + threadIdx.x;
-    uint4 e[OPEN_ROWS_PER_THREAD];
-#pragma unroll
-    for (int k = 0; k < OPEN_ROWS_PER_THREAD; k++) {
-        const uint64_t r = row0 + (uint64_t)k * 256;
-        e[k] = r < job.h ? __ldg(reinterpret_cast<const uint4*>(eq + 4 * r)) : make_uint4(0, 0, 0, 0);
-    }
-    __shared__ uint32_t red[8][4];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    uint32_t* outp = partial + (job.part_off + (uint64_t)chunk * job.w) * 4;
-    for (uint32_t c = 0; c < job.w; c++) {
-        const uint32_t* col = job.cols + (uint64_t)c * job.h;
-        uint32_t a0 = 0, a1 = 0, a2 = 0, a3 = 0;
-#pragma unroll
-        for (int k4 = 0; k4 < OPEN_ROWS_PER_THREAD; k4 += 4) {
-            uint64_t s0 = 0, s1 = 0, s2 = 0, s3 = 0;
-#pragma unroll
-            for (int k = k4; k < k4 + 4; k++) {
-                const uint64_t r = row0 + (uint64_t)k * 256;
-                const uint32_t x = r < job.h ? __ldg(col + r) : 0u;
-                s0 = kb::mac(x, e[k].x, s0); s1 = kb::mac(x, e[k].y, s1); s2 = kb::mac(x, e[k].z, s2); s3 = kb::mac(x, e[k].w, s3);
-            }
-            a0 = kb::add(a0, kb::monty_reduce2(s0)); a1 = kb::add(a1, kb::monty_reduce2(s1));
-            a2 = kb::add(a2, kb::monty_reduce2(s2)); a3 = kb::add(a3, kb::monty_reduce2(s3));
-        }
-        for (int sft = 16; sft > 0; sft >>= 1) {
-            a0 = kb::add(a0, __shfl_down_sync(0xffffffffu, a0, sft)); a1 = kb::add(a1, __shfl_down_sync(0xffffffffu, a1, sft));
-            a2 = kb::add(a2, __shfl_down_sync(0xffffffffu, a2, sft)); a3 = kb::add(a3, __shfl_down_sync(0xffffffffu, a3, sft));
-        }
-        __syncthreads();  // previous column's red[] has been consumed
-        if (lane == 0) { red[warp][0] = a0; red[warp][1] = a1; red[warp][2] = a2; red[warp][3] = a3; }
-        __syncthreads();
-        if (threadIdx.x < 4) {
-            uint32_t v = 0;
-            for (int w = 0; w < 8; w++) v = kb::add(v, red[w][threadIdx.x]);
-            outp[4 * c + threadIdx.x] = v;
-        }
-    }
-}
-// out[(job.out_col + c)] = sum over the table's chunks; one block per table, thread -> (column, limb)
-__global__ void __launch_bounds__(256) gkr_open_reduce_kernel(const OpenJob* __restrict__ jobs, const uint32_t* __restrict__ partial,
-                                                              uint32_t* __restrict__ out) {
-    const OpenJob job = jobs[blockIdx.x];
-    for (uint32_t t = threadIdx.x; t < job.w * 4; t += blockDim.x) {
-        uint32_t v = 0;
-        for (uint32_t b = 0; b < job.nblk; b++) v = kb::add(v, partial[(job.part_off + (uint64_t)b * job.w) * 4 + t]);
-        out[(uint64_t)job.out_col * 4 + t] = v;
-    }
-}
-
 // every read is bounds-checked against the end of the blob and every column against the chip's widths: a blob exported for another
 // chip set must become an error, not an out-of-bounds read on host or device
 const uint32_t* parse_vcol(const uint32_t* b, const uint32_t* end, HostInteractions& H, uint32_t main_w, uint32_t prep_w) {

@@ -39,31 +39,6 @@ void host_compress(const uint32_t* l, const uint32_t* r, uint32_t* out8) {
     for (int j = 0; j < 8; j++) out8[j] = st[j];
 }
 
-// per-column claims: out[c] = sum_{r < rows} row_eq[r] * col[r]   (one block per column)
-__global__ void __launch_bounds__(256) column_claims_kernel(const uint32_t* __restrict__ dense, const uint64_t* __restrict__ col_start,
-                                                            const uint64_t* __restrict__ col_rows, const uint32_t* __restrict__ row_eq,
-                                                            uint32_t* __restrict__ out) {
-    const uint64_t c = blockIdx.x;
-    const uint32_t* col = dense + col_start[c];
-    const uint64_t rows = col_rows[c];
-    uint32_t a0 = 0, a1 = 0, a2 = 0, a3 = 0;
-    for (uint64_t i = threadIdx.x; i < rows; i += blockDim.x) {
-        uint32_t x = __ldg(col + i);
-        uint4 v = __ldg(reinterpret_cast<const uint4*>(row_eq + 4 * i));
-        a0 = kb::add(a0, kb::mul(x, v.x)); a1 = kb::add(a1, kb::mul(x, v.y));
-        a2 = kb::add(a2, kb::mul(x, v.z)); a3 = kb::add(a3, kb::mul(x, v.w));
-    }
-    __shared__ uint32_t red[4][256];
-    red[0][threadIdx.x] = a0; red[1][threadIdx.x] = a1; red[2][threadIdx.x] = a2; red[3][threadIdx.x] = a3;
-    __syncthreads();
-    for (int s = 128; s > 0; s >>= 1) {
-        if ((int)threadIdx.x < s)
-            for (int l = 0; l < 4; l++) red[l][threadIdx.x] = kb::add(red[l][threadIdx.x], red[l][threadIdx.x + s]);
-        __syncthreads();
-    }
-    if (threadIdx.x < 4) out[c * 4 + threadIdx.x] = red[threadIdx.x][0];
-}
-
 // jagged little polynomial: ext[i] = col_eq[c(i)] * row_eq[i - prefix[c(i)]] for i < prefix[ncols], else 0.
 // c(i) = the last column with prefix[c] <= i (zero-height columns share a prefix value: the last one has the non-empty range).
 // start[i >> JP_SHIFT] (built on the host from the same prefix sums) is a column at or before c(i), so the search is a short
@@ -246,82 +221,6 @@ __device__ __forceinline__ int bp_transition(int row_bit, int index_bit, int cur
     return (s >> 1) + 2 * new_cmp;
 }
 
-// One thread per (merged prefix sum k, node in {0, 1/2}).  Point of thread (k, node), big-endian, length dim = 2*(lm+1):
-//   [ bits[k][0 .. split) , lambda , rhos[0 .. round) ]   with split = dim - round - 1
-// left half = "prefix_sum", right half = "next_prefix_sum"; layer l reads the l-th least significant coordinate of each.
-// ri_eq: per layer the 4 values eq((z_row_l, z_index_l), (a, b)) for (a,b) = 00,01,10,11  (shared by all threads).
-// has_lambda == 0: the point is the boolean prefix sums themselves (split == dim): full evaluation, weight zc only.
-__global__ void __launch_bounds__(128) bp_round_kernel(const uint8_t* __restrict__ bits, uint32_t nk, uint32_t dim, uint32_t split,
-                                                       int has_lambda, const uint32_t* __restrict__ rhos, const uint32_t* __restrict__ ri_eq,
-                                                       const uint32_t* __restrict__ zc, const uint32_t* __restrict__ inter, Ext half,
-                                                       uint32_t* __restrict__ partial) {
-    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    Ext v = kb::ext_zero();
-    const uint32_t k = t >> 1, node = t & 1;
-    const uint32_t hl = dim / 2;  // lm + 1
-    if (k < nk && (has_lambda || node == 0)) {
-        const uint8_t* b = bits + (size_t)k * dim;
-        auto coord = [&](uint32_t pos) -> Ext {  // pos in [0, dim)
-            if (pos < split) return b[pos] ? kb::ext_one() : kb::ext_zero();
-            if (has_lambda && pos == split) return node ? half : kb::ext_zero();
-            return kb::ext_load(rhos + 4 * (pos - split - 1));
-        };
-        Ext res[4] = {kb::ext_zero(), kb::ext_zero(), kb::ext_one(), kb::ext_zero()};  // success = carry 0, cmp 1
-        for (int layer = (int)hl; layer >= 0; layer--) {
-            // num_vars = hl (z_index has lm+1 coordinates); layer == hl reads beyond every point -> all coordinates 0
-            Ext cur = kb::ext_zero(), nxt = kb::ext_zero();
-            Ext r00 = kb::ext_one(), r01 = kb::ext_zero(), r10 = kb::ext_zero(), r11 = kb::ext_zero();
-            if ((uint32_t)layer < hl) {
-                cur = coord(hl - 1 - layer);
-                nxt = coord(dim - 1 - layer);
-                const uint32_t* e = ri_eq + (size_t)layer * 16;
-                r00 = kb::ext_load(e); r01 = kb::ext_load(e + 4); r10 = kb::ext_load(e + 8); r11 = kb::ext_load(e + 12);
-            }
-            // eq over (cur, next): c00, c01, c10, c11
-            Ext cn = kb::ext_mul(cur, nxt);
-            Ext c11 = cn, c10 = kb::ext_sub(cur, cn), c01 = kb::ext_sub(nxt, cn);
-            Ext c00 = kb::ext_sub(kb::ext_sub(kb::ext_one(), cur), c01);
-            const Ext ri[4] = {r00, r01, r10, r11};
-            const Ext cc[4] = {c00, c01, c10, c11};
-            Ext nres[4];
-#pragma unroll
-            for (int st = 0; st < 4; st++) {
-                Ext acc = kb::ext_zero();
-#pragma unroll
-                for (int a = 0; a < 4; a++) {      // (row_bit, index_bit)
-                    Ext inner = kb::ext_zero();
-                    bool any = false;
-#pragma unroll
-                    for (int c = 0; c < 4; c++) {  // (cur_bit, next_bit)
-                        int o = bp_transition(a >> 1, a & 1, c >> 1, c & 1, st);
-                        if (o >= 0) { inner = kb::ext_add(inner, kb::ext_mul(cc[c], res[o])); any = true; }
-                    }
-                    if (any) acc = kb::ext_add(acc, kb::ext_mul(ri[a], inner));
-                }
-                nres[st] = acc;
-            }
-#pragma unroll
-            for (int st = 0; st < 4; st++) res[st] = nres[st];
-        }
-        // eq factor of this round's variable and the accumulated one
-        v = kb::ext_mul(kb::ext_load(zc + 4 * k), res[0]);
-        if (has_lambda) {
-            Ext eqv = node ? half : (b[split] ? kb::ext_zero() : kb::ext_one());
-            v = kb::ext_mul(v, kb::ext_mul(kb::ext_load(inter + 4 * k), eqv));
-        }
-    }
-    // block reduce: node 0 -> y_0, node 1 -> y_half
-    __shared__ uint32_t red[4][128];
-    for (int l = 0; l < 4; l++) red[l][threadIdx.x] = v.c[l];
-    __syncthreads();
-    for (int s = 64; s >= 2; s >>= 1) {  // keep parity (node) separate: stop at 2
-        if ((int)threadIdx.x < s)
-            for (int l = 0; l < 4; l++) red[l][threadIdx.x] = kb::add(red[l][threadIdx.x], red[l][threadIdx.x + s]);
-        __syncthreads();
-    }
-    if (threadIdx.x < 8) partial[blockIdx.x * 8 + threadIdx.x] = red[threadIdx.x & 3][threadIdx.x >> 2];
-}
-
 // ---- prefix / suffix form of the same evaluation -----------------------------------------------------------------
 // The evaluation is  e0^T M_0 M_1 ... M_hl init  with one 4x4 transfer matrix per layer, M_l = M(cur_l, next_l).  In sumcheck
 // round r only ONE layer holds the free variable: layers above it still see the column's boolean prefix-sum bits (and, in
@@ -341,7 +240,7 @@ __device__ __forceinline__ void bp_layer_coeffs(const uint32_t* __restrict__ ri_
     m.cc[3] = cn; m.cc[2] = kb::ext_sub(cur, cn); m.cc[1] = kb::ext_sub(nxt, cn);
     m.cc[0] = kb::ext_sub(kb::ext_sub(kb::ext_one(), cur), m.cc[1]);
 }
-// out = M res   (column form; same accumulation order as bp_round_kernel)
+// out = M res   (column form)
 __device__ __forceinline__ void bp_apply(const BpMat& m, const Ext res[4], Ext out[4]) {
 #pragma unroll
     for (int st = 0; st < 4; st++) {
@@ -431,16 +330,8 @@ __global__ void __launch_bounds__(128) bp_round2_kernel(const uint8_t* __restric
         const Ext eqv = node ? half : (b[split] ? kb::ext_zero() : kb::ext_one());
         v = kb::ext_mul(kb::ext_mul(kb::ext_load(zc + 4 * k), val), kb::ext_mul(kb::ext_load(inter + 4 * k), eqv));
     }
-    __shared__ uint32_t red[4][128];
-    for (int l = 0; l < 4; l++) red[l][threadIdx.x] = v.c[l];
-    __syncthreads();
-    for (int s = 64; s >= 2; s >>= 1) {  // keep parity (node) separate: stop at 2
-        if ((int)threadIdx.x < s)
-            for (int l = 0; l < 4; l++) red[l][threadIdx.x] = kb::add(red[l][threadIdx.x], red[l][threadIdx.x + s]);
-        __syncthreads();
-    }
-    if (threadIdx.x < 8) partial[blockIdx.x * 8 + threadIdx.x] = red[threadIdx.x & 3][threadIdx.x >> 2];
-    sp1_mail_done(mail);
+    // per block: the sum at node 0 (y_0), then at node 1 (y_half)
+    block_post_sums<2>({node ? kb::ext_zero() : v, node ? v : kb::ext_zero()}, partial, mail);
 }
 // after round r's challenge: bind position split = dim-1-r: rho_by_pos, inter[k] *= eq(alpha, bit), P_k <- P_k M_layer(bound)
 // (at the switch to the second half P_k restarts at e0^T: the caller rebuilds T with the bound next-coordinates first)
@@ -542,23 +433,22 @@ sp1b200_err sp1b200_jagged_column_claims(sp1b200_ctx* ctx, const sp1b200_jagged_
     const uint32_t mlr = ctx->params.max_log_row_count;
     DevFree mem(ctx);
     uint32_t *d_z, *d_eq, *d_out;
-    uint64_t *d_start, *d_rows;
-    std::vector<uint64_t> start, nrows;
+    // the real tables (the two padding entries at the end excluded), back to back in d_dense
+    std::vector<ColTable> tables;
     uint64_t off = 0;
-    for (size_t t = 0; t + 2 < r->row_counts.size(); t++)
-        for (uint64_t c = 0; c < r->col_counts[t]; c++) { start.push_back(off); nrows.push_back(r->row_counts[t]); off += r->row_counts[t]; }
-    const size_t nc = start.size();
+    size_t nc = 0;
+    for (size_t t = 0; t + 2 < r->row_counts.size(); t++) {
+        tables.push_back(ColTable{r->d_dense + off, r->row_counts[t], (uint32_t)r->col_counts[t], (uint32_t)nc});
+        off += r->row_counts[t] * r->col_counts[t];
+        nc += r->col_counts[t];
+    }
     if (!nc) return nullptr;
     SP1_TRY(mem.alloc((void**)&d_z, mlr * 16));
     SP1_TRY(mem.alloc((void**)&d_eq, ((size_t)16) << mlr));
     SP1_TRY(mem.alloc((void**)&d_out, nc * 16));
-    SP1_TRY(mem.alloc((void**)&d_start, nc * 8));
-    SP1_TRY(mem.alloc((void**)&d_rows, nc * 8));
     SP1_CUDA(cudaMemcpyAsync(d_z, h_z_row, mlr * 16, cudaMemcpyHostToDevice, ctx->stream));
-    SP1_CUDA(cudaMemcpyAsync(d_start, start.data(), nc * 8, cudaMemcpyHostToDevice, ctx->stream));
-    SP1_CUDA(cudaMemcpyAsync(d_rows, nrows.data(), nc * 8, cudaMemcpyHostToDevice, ctx->stream));
     SP1_LAUNCH(ctx, eq_table_kernel, blocks_for((uint64_t)1 << mlr), 256, 0, d_z, (int)mlr, d_eq);
-    SP1_LAUNCH(ctx, column_claims_kernel, (unsigned)nc, 256, 0, r->d_dense, d_start, d_rows, d_eq, d_out);
+    SP1_TRY(column_evals(ctx, mem, tables, d_eq, nc, d_out));
     SP1_CUDA(cudaMemcpyAsync(h_out, d_out, nc * 16, cudaMemcpyDeviceToHost, ctx->stream));
     SP1_CUDA(cudaStreamSynchronize(ctx->stream));
     return nullptr;
@@ -638,7 +528,6 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
     // factored round 0 (no materialised little polynomial) whenever every column starts at an even index
     bool factored = lm >= 2;
     for (uint64_t p : prefix) factored = factored && (p & 1) == 0;
-    { static const bool off = [] { const char* e = getenv("SP1B200_JAGGED_MATERIALISE"); return e && e[0] == '1'; }(); if (off) factored = false; }
     uint32_t* d_roweq2 = nullptr;
     if (factored) {
         SP1_TRY(mem.alloc((void**)&d_ext, (N / 4 + 1) * 16));          // only from round 2 on
@@ -722,7 +611,7 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
 
     // ---- jagged evaluation (branching program) sumcheck --------------------------------------------------------------
     SumcheckProof je;
-    E4 je_claimed[2], je_eval;
+    E4 je_claimed, je_eval;
     {
         PhaseTimer t(ctx, "jagged.eval_sumcheck");
         const uint32_t dim = 2 * (lm + 1);
@@ -747,12 +636,11 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
             E4 e11 = p, e10 = zr - p, e01 = zi - p, e00 = one - zr - e01;
             e00.store(&ri[l * 16]); e01.store(&ri[l * 16 + 4]); e10.store(&ri[l * 16 + 8]); e11.store(&ri[l * 16 + 12]);
         }
-        uint8_t* d_bits; uint32_t *d_ri, *d_zc, *d_inter, *d_rhos, *d_part;
+        uint8_t* d_bits; uint32_t *d_ri, *d_zc, *d_inter, *d_part;
         SP1_TRY(mem.alloc((void**)&d_bits, bits.size()));
         SP1_TRY(mem.alloc((void**)&d_ri, ri.size() * 4));
         SP1_TRY(mem.alloc((void**)&d_zc, (size_t)nk * 16));
         SP1_TRY(mem.alloc((void**)&d_inter, (size_t)nk * 16));
-        SP1_TRY(mem.alloc((void**)&d_rhos, (size_t)dim * 16));
         const unsigned nblk = (2 * nk + 127) / 128;
         SP1_TRY(mem.alloc((void**)&d_part, (size_t)nblk * 32));
         SP1_CUDA(cudaMemcpyAsync(d_bits, bits.data(), bits.size(), cudaMemcpyHostToDevice, st));
@@ -762,11 +650,6 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
         SP1_CUDA(cudaMemcpyAsync(d_inter, ones.data(), (size_t)nk * 16, cudaMemcpyHostToDevice, st));
         const E4 half = E4::from_base(hf::inv(hf::to_monty(2)));
         const Ext dhalf = to_ext(half);
-        // claimed sum = full evaluation at the boolean prefix sums (full_jagged_little_polynomial_evaluation, poly.rs:183-232)
-        SP1_LAUNCH(ctx, bp_round_kernel, nblk, 128, 0, d_bits, nk, dim, dim, 0, d_rhos, d_ri, d_zc, d_inter, dhalf, d_part);
-        SP1_TRY(sum_partials(ctx, d_part, nblk, je_claimed));
-        ch.observe_n(je_claimed[0].c, 4);
-        E4 cl = je_claimed[0];
         // prefix / suffix states (see bp_suffix_kernel): T for the first half now, rebuilt once when the second half starts
         uint32_t *d_T, *d_P, *d_rho_pos;
         SP1_TRY(mem.alloc((void**)&d_T, (size_t)(hl + 2) * nk * 64));
@@ -779,6 +662,16 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
             SP1_CUDA(cudaMemsetAsync(d_rho_pos, 0, (size_t)dim * 16, st));
         }
         SP1_LAUNCH(ctx, bp_suffix_kernel, blocks_for(nk, 128), 128, 0, d_bits, nk, dim, 0, d_rho_pos, d_ri, d_T);
+        // claimed sum = full evaluation at the boolean prefix sums (full_jagged_little_polynomial_evaluation, poly.rs:183-232):
+        // the first-half suffix table reads exactly those bits, so column k evaluates to T_k[0][0]
+        {
+            std::vector<uint32_t> t0((size_t)nk * 16);
+            SP1_CUDA(cudaMemcpyAsync(t0.data(), d_T, t0.size() * 4, cudaMemcpyDeviceToHost, st));
+            SP1_CUDA(cudaStreamSynchronize(st));
+            for (uint32_t k = 0; k < nk; k++) je_claimed = je_claimed + zc[k] * E4::load(&t0[16 * k]);
+        }
+        ch.observe_n(je_claimed.c, 4);
+        E4 cl = je_claimed;
         const bool bp_mail = (size_t)nblk * 8 <= SP1_MAIL_WORDS;  // otherwise fall back to copy + synchronise
         for (uint32_t round = 0; round < dim; round++) {
             if (round == hl) SP1_LAUNCH(ctx, bp_suffix_kernel, blocks_for(nk, 128), 128, 0, d_bits, nk, dim, 1, d_rho_pos, d_ri, d_T);
@@ -813,7 +706,7 @@ sp1b200_err sp1b200_jagged_prove(sp1b200_ctx* ctx, sp1b200_jagged_round* const* 
     auto put = [&](const uint32_t* p, size_t n) { proof.insert(proof.end(), p, p + n); };
     auto put1 = [&](uint32_t v) { proof.push_back(v); };
     sc.emit(proof, claim, round_claim);
-    je.emit(proof, je_claimed[0], je_eval);
+    je.emit(proof, je_claimed, je_eval);
     for (uint32_t r = 0; r < n_rounds; r++) {
         put1((uint32_t)rounds[r]->row_counts.size());
         for (size_t t = 0; t < rounds[r]->row_counts.size(); t++) { put1((uint32_t)rounds[r]->row_counts[t]); put1((uint32_t)rounds[r]->col_counts[t]); }

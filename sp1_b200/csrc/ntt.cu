@@ -14,7 +14,6 @@
 // Step B runs in place on the step-A output of the same column group while it is still L2-resident
 // (B200: 126 MB L2; one 2^23-row column is 32 MB), so the intermediate never costs an HBM round trip.
 #include "ctx.cuh"
-#include <cstdlib>
 #include "kb31.cuh"
 
 namespace {
@@ -319,15 +318,13 @@ sp1b200_err sp1b200_rs_encode_device(sp1b200_ctx* ctx, const uint32_t* d_msg, ui
     int threadsB = (1 << L2) / 2;
     if (threadsB > 1024) threadsB = 1024;
     if (threadsB < 32) threadsB = 32;
-    const bool fast = (L2 == 11) && !ctx->force_generic_ntt;
+    const bool fast = L2 == 11;
     for (uint64_t c0 = 0; c0 < ncols; c0 += group) {
         unsigned nc = (unsigned)((ncols - c0 < group) ? (ncols - c0) : group);
         dim3 gA((1u << L2) / T, nc), gB(1u << (L1 + b), nc);
         // two 1024-thread blocks per SM (32 registers, 9 words of spill) measured 7.42 ms against 7.79 ms for the 52-register build on
-        // the 95 columns of S2 (profiles/bench_r02_occ*.json); SP1B200_RS_A_OCC2=0 selects the one-block build
-        static const bool occ2 = [] { const char* e = getenv("SP1B200_RS_A_OCC2"); return !(e && e[0] == '0'); }();
-        if (fast && L1 == 10 && occ2) SP1_TRY((launch_step_a_fast<10, 2>(ctx, d_msg + c0 * n, d_out + c0 * M, L2, b, nc)));
-        else if (fast && L1 == 10) SP1_TRY(launch_step_a_fast<10>(ctx, d_msg + c0 * n, d_out + c0 * M, L2, b, nc));
+        // the 95 columns of S2 (profiles/bench_r02_occ*.json)
+        if (fast && L1 == 10) SP1_TRY((launch_step_a_fast<10, 2>(ctx, d_msg + c0 * n, d_out + c0 * M, L2, b, nc)));
         else if (fast && L1 == 7) SP1_TRY(launch_step_a_fast<7>(ctx, d_msg + c0 * n, d_out + c0 * M, L2, b, nc));
         else SP1_LAUNCH(ctx, rs_step_a_generic, gA, threadsA, smemA, d_msg + c0 * n, d_out + c0 * M, L1, L2, b, T, ctx->d_TH, ctx->d_TL);
         if (fast) SP1_LAUNCH(ctx, rs_step_b_2048, gB, 256, 0, d_out + c0 * M, L1, b, ctx->d_TH, ctx->d_TL);

@@ -65,42 +65,6 @@ __global__ void __launch_bounds__(256) batch_columns_kernel(const uint32_t* __re
     *reinterpret_cast<uint4*>(out + 4 * i) = make_uint4(a0, a1, a2, a3);
 }
 
-// per-column evaluations at the stack point: evals[c] = sum_i E[i] * cols[c][i]; one block per (column, slice)
-__global__ void __launch_bounds__(256) column_evals_kernel(const uint32_t* __restrict__ cols, uint64_t h, const uint32_t* __restrict__ E,
-                                                           uint32_t* __restrict__ partial, int slices) {
-    const uint64_t c = blockIdx.y;
-    const int sl = blockIdx.x;
-    const uint64_t per = h / slices;
-    const uint32_t* col = cols + c * h + sl * per;
-    const uint32_t* e = E + 4 * (sl * per);
-    uint32_t a0 = 0, a1 = 0, a2 = 0, a3 = 0;
-    for (uint64_t i = threadIdx.x; i < per; i += blockDim.x) {
-        uint32_t x = __ldg(col + i);
-        uint4 v = __ldg(reinterpret_cast<const uint4*>(e + 4 * i));
-        a0 = kb::add(a0, kb::mul(x, v.x)); a1 = kb::add(a1, kb::mul(x, v.y));
-        a2 = kb::add(a2, kb::mul(x, v.z)); a3 = kb::add(a3, kb::mul(x, v.w));
-    }
-    __shared__ uint32_t red[4][256];
-    red[0][threadIdx.x] = a0; red[1][threadIdx.x] = a1; red[2][threadIdx.x] = a2; red[3][threadIdx.x] = a3;
-    __syncthreads();
-    for (int s = 128; s > 0; s >>= 1) {
-        if ((int)threadIdx.x < s)
-            for (int l = 0; l < 4; l++) red[l][threadIdx.x] = kb::add(red[l][threadIdx.x], red[l][threadIdx.x + s]);
-        __syncthreads();
-    }
-    if (threadIdx.x < 4) partial[(c * slices + sl) * 4 + threadIdx.x] = red[threadIdx.x][0];
-}
-
-// out[c] = sum_sl partial[c][sl]
-__global__ void sum_partials_kernel(const uint32_t* __restrict__ partial, int slices, uint64_t n, uint32_t* __restrict__ out) {
-    uint64_t c = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (c >= n) return;
-    uint32_t a[4] = {0, 0, 0, 0};
-    for (int s = 0; s < slices; s++)
-        for (int l = 0; l < 4; l++) a[l] = kb::add(a[l], partial[(c * slices + s) * 4 + l]);
-    for (int l = 0; l < 4; l++) out[4 * c + l] = a[l];
-}
-
 // Ext AoS [h] -> limb-major [4][h]
 __global__ void split_limbs_kernel(const uint32_t* __restrict__ aos, uint64_t h, uint32_t* __restrict__ limbs) {
     uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -118,15 +82,7 @@ __global__ void __launch_bounds__(256) dot_even_kernel(const uint32_t* __restric
         Ext m = kb::ext_load(mle + 8 * j);
         acc = kb::ext_add(acc, kb::ext_mul(e, m));
     }
-    __shared__ uint32_t red[4][256];
-    for (int l = 0; l < 4; l++) red[l][threadIdx.x] = acc.c[l];
-    __syncthreads();
-    for (int s = 128; s > 0; s >>= 1) {
-        if ((int)threadIdx.x < s)
-            for (int l = 0; l < 4; l++) red[l][threadIdx.x] = kb::add(red[l][threadIdx.x], red[l][threadIdx.x + s]);
-        __syncthreads();
-    }
-    if (threadIdx.x < 4) partial[blockIdx.x * 4 + threadIdx.x] = red[threadIdx.x][0];
+    block_post_sums<1>({acc}, partial, Mail{});  // the FRI tree launch that follows posts the round's mail
 }
 
 // mle'[j] = mle[2j] + beta * mle[2j+1]
@@ -277,17 +233,15 @@ sp1b200_err sp1b200_stacked_prove(sp1b200_ctx* ctx, sp1b200_commit* const* round
     for (uint32_t r = 0; r < n_rounds; r++) total_cols += rounds[r]->ncols;
     std::vector<uint32_t> evals(total_cols * 4);
     {
-        const int slices = h >= 4096 ? 16 : 1;
-        uint32_t *d_part, *d_ev;
-        SP1_TRY(mem.alloc((void**)&d_part, total_cols * slices * 16));
-        SP1_TRY(mem.alloc((void**)&d_ev, total_cols * 16));
+        std::vector<ColTable> tables;
         uint64_t off = 0;
         for (uint32_t r = 0; r < n_rounds; r++) {
-            dim3 g(slices, (unsigned)rounds[r]->ncols);
-            SP1_LAUNCH(ctx, column_evals_kernel, g, 256, 0, rounds[r]->d_mles, h, d_E, d_part + off * slices * 4, slices);
+            tables.push_back(ColTable{rounds[r]->d_mles, h, (uint32_t)rounds[r]->ncols, (uint32_t)off});
             off += rounds[r]->ncols;
         }
-        SP1_LAUNCH(ctx, sum_partials_kernel, blocks_for(total_cols), 256, 0, d_part, slices, total_cols, d_ev);
+        uint32_t* d_ev;
+        SP1_TRY(mem.alloc((void**)&d_ev, total_cols * 16));
+        SP1_TRY(column_evals(ctx, mem, tables, d_E, total_cols, d_ev));
         SP1_CUDA(cudaMemcpyAsync(evals.data(), d_ev, total_cols * 16, cudaMemcpyDeviceToHost, st));
         SP1_CUDA(cudaStreamSynchronize(st));
     }

@@ -66,6 +66,107 @@ __device__ __forceinline__ void block_post_sums(const kb::Ext (&v)[N], uint32_t*
     sp1_mail_done(mail);
 }
 
+// index of the job that owns block `blk`: the last one with blk_start <= blk (jobs sorted by blk_start, jobs[0].blk_start = 0)
+template <class J>
+__device__ __forceinline__ int find_job(const J* __restrict__ jobs, int n, uint32_t blk) {
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        int mid = (lo + hi + 1) >> 1;
+        if (jobs[mid].blk_start <= blk) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// ---- per-column evaluations of base-field tables: out[c] = sum_{r < rows} eq[r] * col_c[r] -----------------------------------
+// A block takes one chunk of COL_EVAL_ROWS rows of one table (column-major), keeps its eq values in registers and walks all the
+// table's columns (coalesced column-major reads, 4 products per 64-bit accumulator and reduction); per-column block sums go to
+// partial[(blk_of_table)][col], a second launch adds the chunks.
+constexpr int COL_EVAL_ROWS_PER_THREAD = 16;
+constexpr int COL_EVAL_ROWS = 256 * COL_EVAL_ROWS_PER_THREAD;
+struct ColEvalJob { const uint32_t* cols; uint64_t h; uint32_t w, blk_start, nblk, out_col; uint64_t part_off; };
+
+__global__ void __launch_bounds__(256) column_evals_partial_kernel(const ColEvalJob* __restrict__ jobs, int n_jobs, const uint32_t* __restrict__ eq,
+                                                                   uint32_t* __restrict__ partial) {
+    const ColEvalJob job = jobs[find_job(jobs, n_jobs, blockIdx.x)];
+    const uint32_t chunk = blockIdx.x - job.blk_start;
+    const uint64_t row0 = (uint64_t)chunk * COL_EVAL_ROWS + threadIdx.x;
+    uint4 e[COL_EVAL_ROWS_PER_THREAD];
+#pragma unroll
+    for (int k = 0; k < COL_EVAL_ROWS_PER_THREAD; k++) {
+        const uint64_t r = row0 + (uint64_t)k * 256;
+        e[k] = r < job.h ? __ldg(reinterpret_cast<const uint4*>(eq + 4 * r)) : make_uint4(0, 0, 0, 0);
+    }
+    __shared__ uint32_t red[8][4];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t* outp = partial + (job.part_off + (uint64_t)chunk * job.w) * 4;
+    for (uint32_t c = 0; c < job.w; c++) {
+        const uint32_t* col = job.cols + (uint64_t)c * job.h;
+        uint32_t a0 = 0, a1 = 0, a2 = 0, a3 = 0;
+#pragma unroll
+        for (int k4 = 0; k4 < COL_EVAL_ROWS_PER_THREAD; k4 += 4) {
+            uint64_t s0 = 0, s1 = 0, s2 = 0, s3 = 0;
+#pragma unroll
+            for (int k = k4; k < k4 + 4; k++) {
+                const uint64_t r = row0 + (uint64_t)k * 256;
+                const uint32_t x = r < job.h ? __ldg(col + r) : 0u;
+                s0 = kb::mac(x, e[k].x, s0); s1 = kb::mac(x, e[k].y, s1); s2 = kb::mac(x, e[k].z, s2); s3 = kb::mac(x, e[k].w, s3);
+            }
+            a0 = kb::add(a0, kb::monty_reduce2(s0)); a1 = kb::add(a1, kb::monty_reduce2(s1));
+            a2 = kb::add(a2, kb::monty_reduce2(s2)); a3 = kb::add(a3, kb::monty_reduce2(s3));
+        }
+        for (int sft = 16; sft > 0; sft >>= 1) {
+            a0 = kb::add(a0, __shfl_down_sync(0xffffffffu, a0, sft)); a1 = kb::add(a1, __shfl_down_sync(0xffffffffu, a1, sft));
+            a2 = kb::add(a2, __shfl_down_sync(0xffffffffu, a2, sft)); a3 = kb::add(a3, __shfl_down_sync(0xffffffffu, a3, sft));
+        }
+        __syncthreads();  // previous column's red[] has been consumed
+        if (lane == 0) { red[warp][0] = a0; red[warp][1] = a1; red[warp][2] = a2; red[warp][3] = a3; }
+        __syncthreads();
+        if (threadIdx.x < 4) {
+            uint32_t v = 0;
+            for (int w = 0; w < 8; w++) v = kb::add(v, red[w][threadIdx.x]);
+            outp[4 * c + threadIdx.x] = v;
+        }
+    }
+}
+// out[(job.out_col + c)] = sum over the table's chunks; one block per table, thread -> (column, limb)
+__global__ void __launch_bounds__(256) column_evals_reduce_kernel(const ColEvalJob* __restrict__ jobs, const uint32_t* __restrict__ partial,
+                                                                  uint32_t* __restrict__ out) {
+    const ColEvalJob job = jobs[blockIdx.x];
+    for (uint32_t t = threadIdx.x; t < job.w * 4; t += blockDim.x) {
+        uint32_t v = 0;
+        for (uint32_t b = 0; b < job.nblk; b++) v = kb::add(v, partial[(job.part_off + (uint64_t)b * job.w) * 4 + t]);
+        out[(uint64_t)job.out_col * 4 + t] = v;
+    }
+}
+
+// one table for column_evals: `width` columns of `rows` base-field cells each, column-major at `cols`
+struct ColTable { const uint32_t* cols; uint64_t rows; uint32_t width, out_col; };
+
+// d_out[t.out_col + c] = sum_{r < t.rows} d_eq[r] * column c of t, for every table t, in two launches; d_out holds n_cols ext
+// elements, and the columns of tables without rows (and any column no table names) are zero.
+inline sp1b200_err column_evals(sp1b200_ctx* ctx, DevFree& mem, const std::vector<ColTable>& tables, const uint32_t* d_eq, size_t n_cols,
+                                uint32_t* d_out) {
+    std::vector<ColEvalJob> jobs;
+    uint32_t blk = 0;
+    uint64_t part = 0;
+    for (const ColTable& t : tables) {
+        if (!t.rows) continue;
+        const uint32_t nb = (uint32_t)((t.rows + COL_EVAL_ROWS - 1) / COL_EVAL_ROWS);
+        jobs.push_back(ColEvalJob{t.cols, t.rows, t.width, blk, nb, t.out_col, part});
+        blk += nb; part += (uint64_t)nb * t.width;
+    }
+    SP1_CUDA(cudaMemsetAsync(d_out, 0, n_cols * 16, ctx->stream));
+    if (jobs.empty()) return nullptr;
+    ColEvalJob* d_jobs;
+    uint32_t* d_part;
+    SP1_TRY(mem.alloc((void**)&d_jobs, jobs.size() * sizeof(ColEvalJob)));
+    SP1_TRY(mem.alloc((void**)&d_part, part * 16));
+    SP1_CUDA(cudaMemcpyAsync(d_jobs, jobs.data(), jobs.size() * sizeof(ColEvalJob), cudaMemcpyHostToDevice, ctx->stream));
+    SP1_LAUNCH(ctx, column_evals_partial_kernel, blk, 256, 0, d_jobs, (int)jobs.size(), d_eq, d_part);
+    SP1_LAUNCH(ctx, column_evals_reduce_kernel, (unsigned)jobs.size(), 256, 0, d_jobs, d_part, d_out);
+    return nullptr;
+}
+
 // host side of block_post_sums: waits for the launch with sequence number `seq` and adds up its nblk blocks
 template <int N>
 sp1b200_err mail_sums(sp1b200_ctx* ctx, uint32_t seq, unsigned nblk, hf::E4 (&out)[N]) {

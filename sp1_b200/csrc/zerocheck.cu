@@ -63,16 +63,6 @@ struct ZcFixJob {
     uint32_t main_w, prep_w, blk_start, pad;
 };
 
-template <class J>
-__device__ __forceinline__ int find_job(const J* __restrict__ jobs, int n, uint32_t blk) {
-    int lo = 0, hi = n - 1;
-    while (lo < hi) {
-        int mid = (lo + hi + 1) >> 1;
-        if (jobs[mid].blk_start <= blk) lo = mid; else hi = mid - 1;
-    }
-    return lo;
-}
-
 // register file: every register holds the value at ALL THREE evaluation nodes (the program is decoded once per row pair and
 // the three evaluations run in lockstep: one instruction fetch, three independent products in flight, one pass over the
 // columns).  RF_SMEM: shared memory [reg][node][thread]; RF_LOCAL: a local array (<= 128 registers); RF_GLOBAL: the same
